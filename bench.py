@@ -22,6 +22,10 @@ on the device, max over ranks:
 At N > 1 our arm first runs a numerics self-check (outside the timed regions): 3 steps of a 2-layer model of the
 benchmark's width through the fused NVLink engines and through NCCL + plain kernels; `numerics_ok`, the largest
 relative loss difference and the parameter-checksum difference travel in the JSON line.
+
+`--dump-outputs DIR` (our arm) writes, after the timed regions, what the last timed step computed on rank 0 as
+DIR/<name>.npy (see `dump_outputs`; with --pp > 1 that is the first stage, whose loss is 0).  Weights and token ids are
+seeded, so two builds run with the same arguments get the same inputs and can be compared output for output.
 """
 from __future__ import annotations
 
@@ -62,6 +66,31 @@ def _peak_mem_gb(torch, args):
     except Exception:
         pass
     return None
+
+
+def dump_outputs(out_dir, torch, model, loss):
+    """What the last timed step hands back: ``loss.npy`` (float64 scalar) and ``weights_sample.npy``, the weights after that
+    step's optimizer update (float32, tensors concatenated in ``model.parameters()`` order).  A tensor larger than the
+    per-tensor share of 16 M values (64 MB, at most 16384 a tensor) contributes a sorted sample of positions drawn from a
+    generator seeded with 0, so the same model always yields the same positions.  GPU runs are not bit-reproducible, so
+    compare with a tolerance: two runs of one build (bloom-560m, --gpus 1 --steps 10, B200 at a 1000 W power limit)
+    differed by 7e-5 in the loss and by at most 2.2e-3 in a sampled weight."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array(loss, dtype=np.float64))
+    params = list(model.parameters())
+    per_tensor = max(1, min(16384, (16 << 20) // max(len(params), 1)))
+    gen = torch.Generator().manual_seed(0)
+    parts = []
+    with torch.no_grad():
+        for p in params:
+            flat = p.detach().reshape(-1)
+            if flat.numel() > per_tensor:
+                idx = torch.randint(0, flat.numel(), (per_tensor,), generator=gen).sort().values
+                flat = flat[idx.to(flat.device)]
+            parts.append(flat.float().cpu())
+    np.save(os.path.join(out_dir, "weights_sample.npy"), torch.cat(parts).numpy())
 
 
 class ClockSampler:
@@ -398,6 +427,8 @@ def run_ours(args):
     ms_e2e = timed_region(torch, dist, args.steps, step_e2e)
     if rank == 0:
         sampler.stop()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, torch, model, last["loss"])
     tokens_per_step = args.batch_per_gpu * args.gpus * S
     result = {
         "metric": f"{args.model} training tokens/sec (whole job, device-timed, max over ranks)",
@@ -631,7 +662,13 @@ def main():
                     help="where the random weights are created (auto: on the GPU for the >= 1.7B configs)")
     ap.add_argument("--device", default="cuda", choices=["cuda", "cpu"],
                     help="cpu: dry run of this script on gloo with a tiny model (no benchmark value)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="our arm: write the last timed step's loss and a fixed sample of the updated weights as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs is implemented for --impl ours only")
     args.warmup = max(args.warmup, 3)
     _env_defaults()
     world = int(os.environ["WORLD_SIZE"])

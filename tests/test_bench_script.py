@@ -1,5 +1,7 @@
-"""bench.py is the driver's contract: both arms must run (here: the CPU dry run on gloo with a tiny model), print ONE JSON
-line with the agreed keys, and spell the benchmark configuration identically."""
+"""bench.py's output contract: our arm must run (here: the CPU dry run on gloo with a tiny model), print ONE JSON line with
+the agreed keys, and spell the benchmark configuration exactly as the reference arm does.  The reference is not part of
+this repository, so its side of the comparison is the lines its arm printed on the same arguments, stored under
+tests/golden/."""
 import json
 import os
 import subprocess
@@ -8,15 +10,22 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLDEN = os.path.join(ROOT, "tests", "golden", "bench_reference_arm.json")
 COMMON = ["--device", "cpu", "--model", "bloom-tiny", "--seq-len", "32", "--batch-per-gpu", "2", "--steps", "2", "--warmup", "3"]
 
 
-def _run(extra, env=None):
+def _run(extra):
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + COMMON + extra, capture_output=True, text=True,
-                         timeout=600, cwd=ROOT, env=dict(os.environ, **(env or {})))
+                         timeout=600, cwd=ROOT)
     lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
     assert len(lines) == 1, out.stdout[-2000:] + out.stderr[-2000:]
     return json.loads(lines[0])
+
+
+def _reference_line(extra):
+    """The line ``bench.py --impl reference`` printed for COMMON + ``extra`` with the unmodified reference installed."""
+    with open(GOLDEN) as f:
+        return json.load(f)["lines"][" ".join(extra)]
 
 
 def test_layout_and_config_helpers():
@@ -49,19 +58,37 @@ def test_both_arms_print_one_json_line_with_the_same_config(extra):
     assert ours["e2e"]["h2d_bytes_per_step"] > 0 and ours["e2e"]["d2h_bytes_per_step"] == 4
     if "--hf" in extra:
         return
-    ref = _run(extra + ["--impl", "reference"])
+    ref = _reference_line(extra)
     assert ref["impl"] == "reference"
     assert ref["config"] == ours["config"] and ref["metric"] == ours["metric"]
     if extra[-1] != "1":
         assert ours["numerics_ok"] is True      # the self-check ran (on CPU both engines are the library path)
 
 
+def test_dump_outputs_are_reproducible_and_follow_steps(tmp_path):
+    """``--dump-outputs``: the same arguments give the same outputs; one more timed step gives other weights."""
+    import numpy as np
+
+    dumps = {}
+    for name, steps in (("a", "2"), ("b", "2"), ("c", "3")):
+        line = _run(["--gpus", "1", "--dump-outputs", str(tmp_path / name), "--steps", steps])   # the later --steps wins
+        assert line["steps"] == int(steps)
+        dumps[name] = {f: np.load(tmp_path / name / f) for f in ("loss.npy", "weights_sample.npy")}
+        assert float(dumps[name]["loss.npy"]) == line["final_loss"]
+    a, b, c = dumps["a"], dumps["b"], dumps["c"]
+    assert a["loss.npy"].dtype == np.float64 and a["loss.npy"].shape == ()
+    assert a["weights_sample.npy"].dtype == np.float32 and 0 < a["weights_sample.npy"].nbytes <= 64 << 20
+    for f in a:
+        assert np.array_equal(a[f], b[f]), f
+    assert not np.array_equal(a["weights_sample.npy"], c["weights_sample.npy"])
+
+
 def test_moe_config_both_arms_and_the_reference_arm_in_bf16():
-    """BASELINE.json config #4 shape (Switch-MoE, experts sharded over the tensor group).  The reference arm runs with the
-    model cast to bf16 as on the GPU: its router stays fp32 (it casts its own input), everything else must cope."""
+    """BASELINE.json config #4 shape (Switch-MoE, experts sharded over the tensor group).  The reference arm's line was
+    recorded with the model cast to bf16 as on the GPU: its router stays fp32 (it casts its own input)."""
     extra = ["--gpus", "2", "--tp", "2", "--experts", "2"]
     ours = _run(extra + ["--no-self-check"])
-    ref = _run(extra + ["--impl", "reference"], env={"PIPEGOOSE_B200_BENCH_CPU_BF16": "1"})
+    ref = _reference_line(extra)
     assert ref["impl"] == "reference" and ref["config"] == ours["config"]
     assert ours["config"]["parallelism"] == "tp2dp1+moe2e"
     for line in (ours, ref):
